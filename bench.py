@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (B200 engine)
     python bench.py --impl reference --steps K --warmup W    # reference's CPU path (restated)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last step's output (.npy)
 
 One step = one pass of the hot path over one batch of synthetic input:
 ``transform(table, identity, schema="*", partition=PartitionSpec(by="key", algo="hash", num=256))``
@@ -32,6 +33,9 @@ ALG_BYTES_PER_ROW = 128  # read every column once + write every column once (SUR
 REF_SAMPLE_ROWS = int(os.environ.get("FB_BENCH_REF_ROWS", "1000000"))
 REF_SAMPLE_KEYS = KEY_CARDINALITY * REF_SAMPLE_ROWS // ROWS_PER_GPU
 METRIC = "transform() rows/sec, hash-partitioned (num=256) identity map, 8-col table"
+# --dump-outputs: output rows sampled per column; 13 float64 arrays of 4 MiB (row_index, 4 float64 columns,
+# 4 int64 columns written as two arrays each) plus the partition offsets stay under 64 MB
+DUMP_ROWS = 1 << 19
 
 
 def _peaks():
@@ -58,6 +62,34 @@ def _profile_traffic():
 
 def rows_for(world: int) -> int:
     return ROWS_PER_GPU if world == 1 else ROWS_PER_GPU_DIST
+
+
+def dump_outputs(out, path: str) -> None:
+    """Write the table a ``transform`` call returned as float64 ``.npy`` files under ``path``, so that two
+    builds can be compared output for output: the partition offsets (``offsets``), the positions of a fixed,
+    seeded sample of ``DUMP_ROWS`` output rows (``row_index``; every row when there are fewer) and those rows
+    of every column.  An int64 column becomes two arrays that hold it exactly, ``<name>_hi32`` (signed high
+    32 bits) and ``<name>_lo32`` (low 32 bits)."""
+    import numpy as np
+    import torch
+
+    table = out.native
+    n = table.num_rows
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(table.device)
+    offsets = table.offsets if table.offsets is not None else table.segment_offsets  # multi-GPU: per source rank
+    arrays = {"offsets": offsets.cpu().numpy().ravel().astype(np.float64), "row_index": rows.astype(np.float64)}
+    for name, c in zip(table.schema.names, table.columns):
+        v = c.index_select(0, idx).cpu().numpy()
+        if v.dtype == np.int64:
+            arrays[name + "_hi32"] = (v >> 32).astype(np.float64)
+            arrays[name + "_lo32"] = (v & 0xFFFFFFFF).astype(np.float64)
+        else:
+            assert v.dtype == np.float64, f"{name}: {v.dtype}"
+            arrays[name] = v
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -168,7 +200,7 @@ def run_reference(args):
         return
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
     n = args.rows or rows_for(world)
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     rps, dt = _time_reference(REF_SAMPLE_ROWS, steps, warmup)
     sample = (f"each step = {REF_SAMPLE_ROWS} rows = the logical partitions of {REF_SAMPLE_KEYS} of the "
               f"{KEY_CARDINALITY} keys (same 1526 rows per key as the full workload), restated "
@@ -209,7 +241,7 @@ def run_b200(args):
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     n = args.rows or rows_for(world)
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
 
     # synthetic table of the BASELINE shape, generated on the device, seed = rank
     g = torch.Generator(device=dev).manual_seed(rank)
@@ -262,6 +294,8 @@ def run_b200(args):
     total_rows = n * world
     value = total_rows / (ms_per_step * 1e-3)
     nrows_out = out.count() if hasattr(out, "count") else len(out)
+    if args.dump_outputs:
+        dump_outputs(out, os.path.join(args.dump_outputs, f"rank{rank}") if world > 1 else args.dump_outputs)
     del out
 
     # ---- roofline of the dominant kernel (scatter), timed live with CUDA events on its stream
@@ -440,7 +474,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's output as .npy files under DIR "
+                         "(DIR/rank<r> with several GPUs); see dump_outputs()")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the output of the b200 arm")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,17 +6,12 @@ re-creates only the *shape* of the reference's plugin surface - constructor sign
 plumbing (``EngineFacet``, fugue/execution/execution_engine.py:143-180), ``SQLEngine.encode`` (:202-207),
 the ``conditional_dispatcher`` ``.candidate`` decorators, the registration functions - on top of this repo's
 own host mirror (``fugue_b200.dataframe`` / ``partition`` / ``schema``).  It records every registration so
-the tests can assert what the module registered.  Expression classes: ``install()`` uses the reference's
-real ``fugue/column`` modules when ``/root/reference`` is present (build container), else small
-look-alikes with the same class names and attributes (GPU box).
+the tests can assert what the module registered.  Expression classes: small look-alikes of the reference's
+``fugue/column`` classes with the same class names and attributes.
 """
-import importlib
-import os
 import sys
 import types
-from typing import Any, Dict, List, Optional
-
-REFERENCE_COLUMN_DIR = "/root/reference/fugue/column"
+from typing import Any, Dict, List
 
 
 class Registry:
@@ -26,7 +21,6 @@ class Registry:
         self.candidates: Dict[str, List[Any]] = {}
         self.annotated: Dict[Any, Any] = {}
         self.test_backends: Dict[str, Any] = {}
-        self.reference_ns: Any = None  # the reference's real column DSL (build container only)
 
 
 class _Dispatcher:
@@ -52,9 +46,8 @@ class _Dispatcher:
 
 
 def _lookalike_column_modules() -> Dict[str, types.ModuleType]:
-    """Expression classes with the reference's names and attributes (used only where /root/reference
-    is absent); structure follows fugue/column/expressions.py:8-856 at the level of class names and
-    public properties, nothing more."""
+    """Expression classes with the reference's names and attributes; structure follows
+    fugue/column/expressions.py:8-856 at the level of class names and public properties, nothing more."""
     fe = types.ModuleType("fugue.column.expressions")
     ff = types.ModuleType("fugue.column.functions")
 
@@ -120,7 +113,7 @@ def _lookalike_column_modules() -> Dict[str, types.ModuleType]:
     return {"fugue.column.expressions": fe, "fugue.column.functions": ff}
 
 
-def install(use_reference_column: Optional[bool] = None) -> Registry:
+def install() -> Registry:
     """Put the stand-in modules into ``sys.modules`` (idempotent per process) and return the registry."""
     if "fugue" in sys.modules and hasattr(sys.modules["fugue"], "_standin_registry"):
         return sys.modules["fugue"]._standin_registry
@@ -246,25 +239,12 @@ def install(use_reference_column: Optional[bool] = None) -> Registry:
     mods = {"fugue": fugue, "fugue.dataframe": f_df, "fugue.dataframe.dataframe": f_dfdf, "fugue.dev": f_dev,
             "fugue.execution": f_ex, "fugue.execution.factory": f_fac, "fugue.plugins": f_pl, "fugue.test": f_test,
             "triad": triad}
-    if use_reference_column is None:
-        use_reference_column = os.path.isdir(REFERENCE_COLUMN_DIR)
     sys.modules.update(mods)
-    if use_reference_column:
-        # the reference's real column DSL, loaded by file path with the helper stand-ins of the golden generator
-        sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-        gen = importlib.import_module("make_column_golden")
-        reg.reference_ns = gen._load_reference_column()  # installs fugue.column.{expressions,functions,sql}
-        sys.modules.update(mods)  # ... and its own bare "fugue" / "triad": put ours back
-        fcol = sys.modules["fugue.column"]
-        fugue.column = fcol
-        fcol.expressions = sys.modules["fugue.column.expressions"]
-        fcol.functions = sys.modules["fugue.column.functions"]
-    else:
-        fcol = types.ModuleType("fugue.column")
-        fcol.__path__ = []
-        look = _lookalike_column_modules()
-        sys.modules.update(look)
-        sys.modules["fugue.column"] = fcol
-        fcol.expressions, fcol.functions = look["fugue.column.expressions"], look["fugue.column.functions"]
-        fugue.column = fcol
+    fcol = types.ModuleType("fugue.column")
+    fcol.__path__ = []
+    look = _lookalike_column_modules()
+    sys.modules.update(look)
+    sys.modules["fugue.column"] = fcol
+    fcol.expressions, fcol.functions = look["fugue.column.expressions"], look["fugue.column.functions"]
+    fugue.column = fcol
     return reg

@@ -7,7 +7,9 @@ their real names, with a minimal stand-in for those helpers (Schema / type names
 assert_or_throw - nothing of the DSL logic), builds a catalogue of expressions with the reference classes
 and records what the reference says about each: ``str(expr)``, the SQL its ``SQLExpressionGenerator`` emits,
 the inferred alias and the inferred type.  ``tests/test_column_golden.py`` builds the same catalogue with
-``fugue_b200.column`` and compares.  Run here only (needs /root/reference):
+``fugue_b200.column`` and compares.  The reference's trees themselves go to ``column_dsl_trees.json``, which
+``tests/test_fugue_plugin.py`` rebuilds and runs through the plugin's ``translate_expr``.  Run it where the
+reference's sources are at ``REF``:
 
     python tests/golden/make_column_golden.py
 """
@@ -84,8 +86,26 @@ def _load_reference_column():
     return ns
 
 
+def _tree(e):
+    """A reference expression node as JSON: its class and base classes (``translate_expr`` dispatches on the
+    bases) and the attributes ``translate_expr`` reads.  Plain Python values are stored as ``{"py": value}``."""
+    fe = sys.modules["fugue.column.expressions"]
+    if not isinstance(e, fe.ColumnExpr):
+        return {"py": e}
+    node = {"mro": [c.__name__ for c in type(e).__mro__ if c is not object], "as_name": e.as_name,
+            "as_type": None if e.as_type is None else str(e.as_type)}
+    if isinstance(e, fe._NamedColumnExpr):
+        node["name"] = e.name
+    elif isinstance(e, fe._LiteralColumnExpr):
+        node["value"] = e.value
+    elif isinstance(e, fe._FuncExpr):
+        node.update(func=e.func, args=[_tree(a) for a in e.args], is_distinct=e.is_distinct,
+                    kwargs={k: _tree(v) for k, v in e.kwargs.items()})
+    return node
+
+
 def main() -> None:
-    from column_catalogue import describe_all
+    from column_catalogue import _expressions, describe_all
 
     ns = _load_reference_column()
     out = describe_all(ns)
@@ -93,6 +113,11 @@ def main() -> None:
     with open(path, "w") as fp:
         json.dump(out, fp, indent=1, sort_keys=True)
     print(f"wrote {path}: {len(out['expressions'])} expressions, {len(out['selects'])} selects")
+    trees = {k: _tree(e) for k, e in _expressions(ns).items()}
+    path = os.path.join(HERE, "column_dsl_trees.json")
+    with open(path, "w") as fp:
+        json.dump(trees, fp, indent=1, sort_keys=True)
+    print(f"wrote {path}: {len(trees)} expression trees")
 
 
 if __name__ == "__main__":

@@ -1,7 +1,7 @@
 """``fugue_b200/fugue_plugin.py`` executed against the stand-in of the reference's plugin surface
-(tests/fugue_standin.py): what it registers, and - in the build container, where the reference's own
-``fugue/column`` modules can be loaded - that the reference's expression trees survive the translation
-into the engine's IR (replay of tests/golden/column_dsl_vectors.json through ``translate_expr``).
+(tests/fugue_standin.py): what it registers, and that the reference's expression trees (recorded from its
+own ``fugue/column`` code in tests/golden/column_dsl_trees.json) survive the translation into the engine's
+IR (replay of tests/golden/column_dsl_vectors.json through ``translate_expr``).
 The device half (the adapter's engine running select / aggregate / join / SQL) is in the GPU test below."""
 import json
 import os
@@ -40,20 +40,41 @@ def test_module_registers_engine_sql_engine_candidates_and_test_backend(plugin):
     assert "super().join(" not in src and "super().select(" not in src and "super().aggregate(" not in src  # no host fallback
 
 
-def test_reference_trees_translate_into_the_ir(plugin):
-    reg, mod = plugin
-    if reg.reference_ns is None:
-        pytest.skip("needs /root/reference (build container)")
-    from column_catalogue import _expressions
+def _rebuild(node):
+    """A tree of tests/golden/column_dsl_trees.json, rebuilt with the expression classes under ``fugue.column``;
+    each node takes the first class of its recorded class hierarchy that those modules define."""
+    import pyarrow as pa
 
+    if "py" in node:
+        return node["py"]
+    mods = (sys.modules["fugue.column.expressions"], sys.modules["fugue.column.functions"])
+    cls = next(getattr(m, c) for c in node["mro"] for m in mods if hasattr(m, c))
+    if "name" in node:
+        e = cls(node["name"])
+    elif "value" in node:
+        e = cls(node["value"])
+    elif "func" in node:
+        e = cls(node["func"], *[_rebuild(a) for a in node["args"]], arg_distinct=node["is_distinct"],
+                **{k: _rebuild(v) for k, v in node["kwargs"].items()})
+    else:
+        e = cls()
+    e.as_name = node["as_name"]
+    e.as_type = None if node["as_type"] is None else pa.type_for_alias(node["as_type"])
+    return e
+
+
+def test_reference_trees_translate_into_the_ir(plugin):
+    _, mod = plugin
     from fugue_b200 import column as ir
     from fugue_b200.schema import Schema
 
     want = json.load(open(os.path.join(HERE, "golden", "column_dsl_vectors.json")))["expressions"]
+    trees = json.load(open(os.path.join(HERE, "golden", "column_dsl_trees.json")))
+    assert set(trees) == set(want)
     schema = Schema("a:int,b:long,c:bool,d:double,s:str")
     bad = []
-    for name, ref_tree in _expressions(reg.reference_ns).items():
-        mine = mod.translate_expr(ref_tree)
+    for name, node in trees.items():
+        mine = mod.translate_expr(_rebuild(node))
         got = {"str": str(mine), "is_agg": ir.is_agg(mine), "sql": ir.to_sql(mine)}
         try:
             got["inferred_alias"] = mine.infer_alias().output_name
