@@ -55,12 +55,15 @@ __device__ __forceinline__ uint64_t ordered_to_f64(long long o) {
   return o >= 0 ? (uint64_t)o : ((uint64_t)o ^ 0x7FFFFFFFFFFFFFFFULL);
 }
 
+// The f64 identities are the ends of the ordered code (IEEE total order: -NaN < -inf < ... < +inf < +NaN),
+// not +-inf: MIN over {+NaN} must stay +NaN.  An identity never reaches the output - a group either has a
+// non-NULL value or its hidden COUNT makes the result NULL.
 __device__ __forceinline__ uint64_t identity_of(int op) {
   switch (op) {
-    case kMinI64: return (uint64_t)0x7FFFFFFFFFFFFFFFLL;
-    case kMaxI64: return (uint64_t)0x8000000000000000ULL;
-    case kMinF64: return (uint64_t)f64_to_ordered(0x7FF0000000000000ULL);  // +inf
-    case kMaxF64: return (uint64_t)f64_to_ordered(0xFFF0000000000000ULL);  // -inf
+    case kMinI64:
+    case kMinF64: return (uint64_t)0x7FFFFFFFFFFFFFFFLL;
+    case kMaxI64:
+    case kMaxF64: return (uint64_t)0x8000000000000000ULL;
     default: return 0;  // sums and counts (0.0 == bit pattern 0)
   }
 }

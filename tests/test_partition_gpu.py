@@ -200,16 +200,138 @@ def test_full_size_properties_100m_rows():
     assert int((rid ^ (rid >> 7)).sum()) == int((rowid ^ (rowid >> 7)).sum())
 
 
-@pytest.mark.parametrize("env", [{}, {"FB_SCATTER": "swc"}, {"FB_DISABLE_TMA": "1"}, {"FB_WS_COLS": "8"},
-                                 {"FB_WS_COLS": "1"}])
-def test_all_scatter_kernel_paths_agree(env, monkeypatch):
-    """warp-specialised (default), single-role write-combining (v4) and generic kernels: same bits."""
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
+def _sms() -> int:
+    import ctypes as C
+
+    from fugue_b200 import _lib
+
+    sm, mem, maj, mnr = C.c_int(), C.c_size_t(), C.c_int(), C.c_int()
+    _lib.check(_lib.load().fb_device_info(0, C.byref(sm), C.byref(mem), C.byref(maj), C.byref(mnr)))
+    return sm.value
+
+
+def _check_apply(dcols, key_idx, num, exp, out=None, **kw):
+    """partition_plan + partition_apply(**kw) of the device columns ``dcols`` == ``exp``, the oracle's partition."""
+    from fugue_b200 import kernels as K
+
+    plan = K.partition_plan([dcols[i] for i in key_idx], num)
+    got = K.partition_apply(plan, dcols, out=out, **kw)
+    torch.cuda.synchronize()
+    exp_cols, exp_off = exp
+    assert np.array_equal(plan.offsets.cpu().numpy(), exp_off)
+    for c, (a, b) in enumerate(zip(got, exp_cols)):
+        assert np.array_equal(_bytes(a), np.ascontiguousarray(b).view("u1")), f"column {c} differs ({kw})"
+
+
+@pytest.fixture(scope="module")
+def ten_columns():
     rng = np.random.default_rng(23)
     n = 1_234_567
     cols = [rng.integers(0, 1 << 16, n).astype("int64")] + \
            [rng.integers(-(2**62), 2**62, n).astype("int64") for _ in range(4)] + \
            [rng.standard_normal(n) for _ in range(5)]          # 10 columns: more than one launch
-    _check_partition(cols, [0], 256)
-    _check_partition(cols, [0, 5], 200)                           # two key columns, num not a power of two
+    exp = {(0,): hp.partition_table(cols, [0], 256), (0, 5): hp.partition_table(cols, [0, 5], 200)}
+    return [_to_dev(c) for c in cols], exp
+
+
+@pytest.mark.parametrize("cols_per_launch", [0, 1, 2, 3, 5, 8])
+@pytest.mark.parametrize("ctas", [None, 7, 1], ids=["all-sms", "7-ctas", "1-cta"])
+def test_all_scatter_kernel_paths_agree(ten_columns, cols_per_launch, ctas):
+    """The warp-specialised scatter kernel under every launch shape: ``cols_per_launch`` columns per launch (0 = the
+    default grouping) on a grid cut to ``ctas`` CTAs by ``sm_reserve = sms - ctas``.  With one CTA, that CTA runs
+    every chunk through one mbarrier pipeline (chunk-to-chunk hand-over: flush barrier, look-ahead of the next rank
+    record, carry reset).  One key column at num 256 and two key columns at num 200: same bits as the oracle."""
+    d, exp = ten_columns
+    r = 0 if ctas is None else _sms() - ctas
+    _check_apply(d, [0], 256, exp[(0,)], sm_reserve=r, cols_per_launch=cols_per_launch)
+    _check_apply(d, [0, 5], 200, exp[(0, 5)], sm_reserve=r, cols_per_launch=cols_per_launch)
+
+
+@pytest.mark.parametrize("num", [16, 17])
+@pytest.mark.parametrize("shape", ["chunks+tail", "whole-tiles", "whole-tiles+1"])
+def test_scatter_chunk_geometry(shape, num):
+    """Row counts cut from the SM count at run time (4096-row tiles, at most 2 chunks per SM): 3 * (2 * sms) + 1 whole
+    tiles plus a partial tile (4 tiles per chunk, a last chunk of one tile, a tail); exactly k whole tiles (no tail);
+    k tiles and one row.  num 16 / 17 is the 4-bit / 8-bit boundary of the rank and scatter kernel templates."""
+    sms = _sms()
+    k = 2 * sms + 5
+    n = {"chunks+tail": (3 * (2 * sms) + 1) * 4096 + 2049, "whole-tiles": 4096 * k, "whole-tiles+1": 4096 * k + 1}[shape]
+    rng = np.random.default_rng(n + num)
+    cols = [rng.integers(-(2**62), 2**62, n).astype("int64"), rng.standard_normal(n),
+            rng.integers(-1000, 1000, n).astype("int32"), np.arange(n, dtype="int64"),
+            rng.integers(0, 255, n).astype("uint8")]
+    d = [_to_dev(c) for c in cols]
+    for key_idx in ([0], [0, 2]):
+        exp = hp.partition_table(cols, key_idx, num)
+        for r in (0, sms - 1):
+            _check_apply(d, key_idx, num, exp, sm_reserve=r)
+
+
+def _misaligned(n: int, dtype):
+    """A 1-d tensor of n elements that is 8-byte but not 16-byte aligned."""
+    buf = torch.empty(n + 1, dtype=dtype, device=_dev())
+    t = buf[1:]
+    assert t.is_contiguous() and t.data_ptr() % 16 == 8
+    return t
+
+
+def test_scatter_mixes_aligned_and_misaligned_columns_in_one_call():
+    """8-byte columns at 16-byte aligned addresses go to the warp-specialised kernel, those 8 bytes off to the generic
+    one (and so do narrow columns) - in one call, with some outputs misaligned too."""
+    rng = np.random.default_rng(29)
+    n = 1_000_003
+    cols = [rng.integers(0, 1 << 20, n).astype("int64"), rng.integers(-(2**62), 2**62, n).astype("int64"),
+            rng.standard_normal(n), rng.integers(-(2**62), 2**62, n).astype("int64"), rng.standard_normal(n),
+            rng.integers(-(2**30), 2**30, n).astype("int32")]
+    d = []
+    for i, c in enumerate(cols):
+        t = _to_dev(c)
+        if i in (1, 4):  # misaligned sources
+            m = _misaligned(n, t.dtype)
+            m.copy_(t)
+            t = m
+        d.append(t)
+    assert [t.data_ptr() % 16 for t in d] == [0, 8, 0, 0, 8, 0]
+    out = [torch.empty_like(t) if i in (0, 1, 5) else _misaligned(n, t.dtype) for i, t in enumerate(d)]
+    exp = hp.partition_table(cols, [0], 256)
+    for r in (0, _sms() - 1):
+        _check_apply(d, [0], 256, exp, out=[o.fill_(0) for o in out], sm_reserve=r)
+
+
+def test_fused_map_on_one_cta_with_a_tail_tile():
+    """K4 (partition_apply_map) with 9 units - copies, one- and two-operand affine maps in float64 and wrapping int64 -
+    on a single CTA (sm_reserve = sms - 1), n with a partial tail tile: the numpy epilogue model over the oracle's
+    partition order, bit for bit."""
+    import struct
+
+    from fugue_b200 import kernels as K
+    from test_colmap_plan import _epilogue
+
+    sms = _sms()
+    n = 4096 * (2 * sms + 5) + 1234
+    rng = np.random.default_rng(31)
+    key = rng.integers(0, 1 << 16, n).astype("int64")
+    xs = [rng.standard_normal(n) * 10.0 ** rng.integers(-3, 4, n) for _ in range(3)]
+    js = [rng.integers(-(2**62), 2**62, n).astype("int64"), rng.integers(-1000, 1000, n).astype("int64")]
+    fb = lambda v: struct.unpack("<Q", struct.pack("<d", v))[0]  # noqa: E731
+    host = {f"x{i}": torch.from_numpy(a) for i, a in enumerate(xs)}
+    host.update({f"j{i}": torch.from_numpy(a) for i, a in enumerate(js)})
+    F, I, CP = K.MAP_AFFINE_F64, K.MAP_AFFINE_I64, K.MAP_COPY
+    units = [("x0", None, CP, 0, 0, 0), ("j0", None, CP, 0, 0, 0),
+             ("x0", None, F, fb(2.5), 0, fb(-0.0)), ("x1", "x2", F, fb(-1.25), fb(3.0), fb(0.5)),
+             ("x2", "x0", F, fb(1e-3), fb(-7.0), fb(-2.0)),
+             ("j0", None, I, 3, 0, -7), ("j0", "j1", I, 0x9E3779B97F4A7C15, -5, 11),
+             ("j1", "j0", I, -1, 1, 0), ("x1", None, F, fb(-1.0), 0, fb(0.0))]
+    assert len(units) == 9 and {u[2] for u in units} == {CP, F, I}
+    dev = {k: v.to(_dev()) for k, v in host.items()}
+    dkey = _to_dev(key)
+    plan = K.partition_plan([dkey], 256)
+    got = K.partition_apply_map(plan, [(dev[x], None if y is None else dev[y], m, a, b, c) for x, y, m, a, b, c in units],
+                                sm_reserve=sms - 1)
+    torch.cuda.synchronize()
+    order, off = hp.stable_partition(hp.partition_ids([key], 256), 256)
+    assert np.array_equal(plan.offsets.cpu().numpy(), off)
+    for i, (x, y, m, a, b, c) in enumerate(units):
+        mask = (1 << 64) - 1
+        want = _epilogue((host[x], None if y is None else host[y], m, a & mask, b & mask, c & mask, None), n)[order]
+        assert np.array_equal(got[i].cpu().numpy().view(np.uint64), want), f"unit {i}"
