@@ -87,12 +87,17 @@ FB_HD uint64_t fb_mulhi64(uint64_t a, uint64_t b) {
 #endif
 }
 
-FB_HD uint32_t fb_fastmod(uint64_t n, const FbDiv& dv) {
-  if ((dv.d & (dv.d - 1)) == 0) return (uint32_t)n & (dv.d - 1);  // power of two (and d == 1)
+// d not a power of two
+FB_HD uint32_t fb_fastmod_magic(uint64_t n, const FbDiv& dv) {
   uint64_t q = fb_mulhi64(dv.magic, n);
   uint64_t t = ((n - q) >> 1) + q;
   q = t >> dv.shift;
   return (uint32_t)(n - q * dv.d);
+}
+
+FB_HD uint32_t fb_fastmod(uint64_t n, const FbDiv& dv) {
+  if ((dv.d & (dv.d - 1)) == 0) return (uint32_t)n & (dv.d - 1);  // power of two (and d == 1)
+  return fb_fastmod_magic(n, dv);
 }
 
 // pandas _hash_ndarray finaliser (splitmix64)

@@ -174,75 +174,103 @@ fb_hist_kernel(FbKeys keys, FbDiv dv, uint32_t num, ChunkGeom g, int chunk0, uin
 //   [0, 4096)       uint8  partition id of every row
 //   [4096, 12288)   uint16 rank of the row among the rows of the same partition in this tile
 //   [12288, 12800)  uint16 rows per partition in this tile (256 entries)
-// Pass 2 loads one record per tile with a single TMA bulk copy.  This kernel runs at full occupancy
-// (2 x 1024 threads per SM); the same work done by the 8 ranker warps of the pass-2 CTA was the
-// bottleneck of 4-column launches (profiles/r1_notes.md).
+// Pass 2 loads one record per tile with a single TMA bulk copy.
+//
+// One warp ranks a whole tile, 32 rows per step in row order, against warp-private counters: the
+// rank of a row is the counter of its partition plus the lanes of the same partition below it, so
+// no prefix over warps and no block barrier is needed, and the counters are the tile's counts when
+// the tile ends.  The lanes of the same partition come from kBits ballots turned into two
+// 16-entry lookup tables (lane i holds the lanes whose low / high nibble is not i), read back with
+// two shuffles: one vote and one LOP3 per bit instead of a per-bit select and merge in every lane.
+// The CTA (2 x 1024 threads per SM) owns one chunk; its warps take the chunk's tiles in turn.
 // ---------------------------------------------------------------------------
-constexpr int kRankBlock = 1024, kRankWarps = kRankBlock / 32, kRankItems = kTile / kRankBlock;
+constexpr int kRankBlock = 1024, kRankWarps = kRankBlock / 32;
 constexpr uint32_t kMetaRank = kTile, kMetaCnt = 3 * kTile, kMetaBytes = 3 * kTile + 512;
-static_assert(kRankItems * kRankBlock == kTile, "tile must be a multiple of the rank block");
 
-template <bool kSingleU64, int kBits>
+// ballot of (v & bit) != 0; spelled in PTX so that the test stays one predicate-setting instruction
+__device__ __forceinline__ unsigned ballot_bit(uint32_t v, uint32_t bit) {
+  unsigned r;
+  asm("{\n\t.reg .pred p;\n\t.reg .b32 t;\n\tand.b32 t, %1, %2;\n\tsetp.ne.u32 p, t, 0;\n\t"
+      "vote.sync.ballot.b32 %0, p, 0xffffffff;\n}"
+      : "=r"(r)
+      : "r"(v), "r"(bit));
+  return r;
+}
+
+template <bool kSingleU64, int kBits, bool kPow2>
 __global__ void __launch_bounds__(kRankBlock, 2)
 fb_rank_kernel(FbKeys keys, FbDiv dv, uint32_t num, ChunkGeom g, uint32_t* __restrict__ hist,
                uint8_t* __restrict__ meta) {
-  __shared__ uint16_t s_cnt[kRankWarps * 256];
-  for (uint32_t i = threadIdx.x; i < (uint32_t)kRankWarps * 256; i += kRankBlock) s_cnt[i] = 0;
+  static_assert(kBits == 4 || kBits == 8, "partition ids of 4 or 8 bits");
+  // steps whose keys are loaded together; the 64-bit division by other counts needs the registers
+  constexpr int kUnroll = kSingleU64 && !kPow2 ? 2 : 4;
+  __shared__ __align__(16) uint16_t s_cnt[kRankWarps][256];
+  __shared__ uint32_t s_hist[256];
+  for (uint32_t i = threadIdx.x; i < (uint32_t)kRankWarps * 128; i += kRankBlock) ((uint32_t*)s_cnt)[i] = 0;
+  if (threadIdx.x < 256) s_hist[threadIdx.x] = 0;
   __syncthreads();
   int64_t row0, row1;
   chunk_range(g, (int)blockIdx.x, row0, row1);  // launched over the full chunks only
+  const uint32_t tile0 = (uint32_t)(row0 / kTile), ntiles = (uint32_t)((row1 - row0) / kTile);
   const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const unsigned lt = fb_lanemask_lt();
-  uint16_t* __restrict__ my = s_cnt + warp * 256;
-  uint32_t acc = 0;  // thread b < num: rows of partition b in this chunk
-  for (int64_t t0 = row0; t0 < row1; t0 += kTile) {
-    uint8_t* __restrict__ rec = meta + (size_t)(t0 / kTile) * kMetaBytes;
-    uint32_t pid[kRankItems], pos[kRankItems];
+  uint16_t* __restrict__ my = s_cnt[warp];
+  unsigned neg[4];  // lane i, table entry i & 15: bit b of i spread over the word
 #pragma unroll
-    for (int r = 0; r < kRankItems; ++r)
-      pid[r] = compute_pid<kSingleU64>(keys, dv, t0 + warp * (32 * kRankItems) + r * 32 + lane);
-    unsigned mm[kRankItems];
+  for (int b = 0; b < 4; ++b) neg[b] = 0u - ((lane >> b) & 1u);
+  for (uint32_t t = tile0 + warp; t < tile0 + ntiles; t += kRankWarps) {
+    const int64_t t0 = (int64_t)t * kTile;
+    uint8_t* __restrict__ rec = meta + (size_t)t * kMetaBytes;
+    uint8_t* __restrict__ rp = rec + lane;
+    uint16_t* __restrict__ rq = (uint16_t*)(rec + kMetaRank) + lane;
+    const uint32_t r0 = (uint32_t)t0 + lane;  // plan_impl limits nrows to 32 bits
+#pragma unroll 1
+    for (int i = 0; i < kTile / 32; i += kUnroll) {
+      uint32_t pid[kUnroll];
 #pragma unroll
-    for (int r = 0; r < kRankItems; ++r) mm[r] = match_lanes<kBits>(pid[r], 0xFFFFFFFFu);
-#pragma unroll
-    for (int r = 0; r < kRankItems; ++r) {
-      const unsigned m = mm[r];
-      const unsigned before = __popc(m & lt);
-      uint32_t old = 0;
-      if (before == 0) {
-        old = my[pid[r]];
-        my[pid[r]] = (uint16_t)(old + __popc(m));
+      for (int u = 0; u < kUnroll; ++u) {
+        if (kSingleU64) {  // compute_pid with the divisor's kind known at compile time
+          const uint64_t h = fb_hash_single_u64(__ldg((const unsigned long long*)keys.ptr[0] + (r0 + (i + u) * 32)));
+          pid[u] = kPow2 ? (uint32_t)h & (dv.d - 1) : fb_fastmod_magic(h, dv);
+        } else {
+          pid[u] = compute_pid<false>(keys, dv, r0 + (i + u) * 32);
+        }
       }
-      __syncwarp();
-      old = __shfl_sync(0xFFFFFFFFu, old, __ffs(m) - 1);
-      pos[r] = old + before;
-    }
-    __syncthreads();
-    if (threadIdx.x < 256) {  // exclusive prefix over the warps, per partition
-      const uint32_t b = threadIdx.x;
-      uint32_t n = 0;
 #pragma unroll
-      for (int w = 0; w < kRankWarps; ++w) {
-        const uint32_t t = s_cnt[w * 256 + b];
-        s_cnt[w * 256 + b] = (uint16_t)n;
-        n += t;
+      for (int u = 0; u < kUnroll; ++u) {
+        const uint32_t p = pid[u];
+        // lo / hi: lanes whose low / high nibble differs from table entry lane & 15
+        unsigned lo = ballot_bit(p, 1) ^ neg[0], hi = kBits > 4 ? ballot_bit(p, 16) ^ neg[0] : 0;
+#pragma unroll
+        for (int b = 1; b < 4; ++b) {
+          lo |= ballot_bit(p, 1u << b) ^ neg[b];
+          if (kBits > 4) hi |= ballot_bit(p, 16u << b) ^ neg[b];
+        }
+        lo = __shfl_sync(0xFFFFFFFFu, lo, p, 16);
+        if (kBits > 4) hi = __shfl_sync(0xFFFFFFFFu, hi, p >> 4, 16);
+        const unsigned m = ~(lo | hi);  // lanes with partition p
+        const uint32_t old = my[p];
+        __syncwarp();
+        my[p] = (uint16_t)(old + __popc(m));  // the same value from every lane of the partition
+        __syncwarp();
+        rp[(i + u) * 32] = (uint8_t)p;
+        rq[(i + u) * 32] = (uint16_t)(old + __popc(m & lt));
       }
-      acc += n;
-      ((uint16_t*)(rec + kMetaCnt))[b] = (uint16_t)n;
     }
-    __syncthreads();
+    // the counters are the tile's counts: lane l moves partitions 8l .. 8l + 7 and clears them
+    const uint4 c = ((const uint4*)my)[lane];
+    ((uint4*)(rec + kMetaCnt))[lane] = c;
+    ((uint4*)my)[lane] = make_uint4(0, 0, 0, 0);
+    const uint32_t w[4] = {c.x, c.y, c.z, c.w};
 #pragma unroll
-    for (int r = 0; r < kRankItems; ++r) {
-      const uint32_t idx = warp * (32 * kRankItems) + r * 32 + lane;
-      rec[idx] = (uint8_t)pid[r];
-      ((uint16_t*)(rec + kMetaRank))[idx] = (uint16_t)(pos[r] + my[pid[r]]);
+    for (int j = 0; j < 4; ++j) {
+      atomicAdd(&s_hist[lane * 8 + 2 * j], w[j] & 0xFFFFu);
+      atomicAdd(&s_hist[lane * 8 + 2 * j + 1], w[j] >> 16);
     }
-    __syncwarp();
-#pragma unroll
-    for (int i = 0; i < 4; ++i) ((uint32_t*)my)[i * 32 + lane] = 0;
     __syncwarp();
   }
-  if (threadIdx.x < num) hist[(size_t)blockIdx.x * num + threadIdx.x] = acc;
+  __syncthreads();
+  if (threadIdx.x < num) hist[(size_t)blockIdx.x * num + threadIdx.x] = s_hist[threadIdx.x];
 }
 
 // ---------------------------------------------------------------------------
@@ -1216,6 +1244,7 @@ static int plan_impl(int dev, void* stream, int64_t nrows, const FbKeys& k, bool
   PlanLayout l = plan_layout(g, num_partitions);
   FB_CHECK(scratch != nullptr && scratch_bytes >= l.total_bytes,
            "scratch too small: need %zu bytes, got %zu", l.total_bytes, scratch_bytes);
+  FB_CHECK((uintptr_t)scratch % 16 == 0, "scratch must be 16-byte aligned (rank records are stored in 16-byte words)");
   FbDiv dv = fb_make_div(num_partitions);
   uint32_t* hist = (uint32_t*)scratch;
   size_t smem = (size_t)kHistWarps * num_partitions * sizeof(uint32_t);
@@ -1226,13 +1255,20 @@ static int plan_impl(int dev, void* stream, int64_t nrows, const FbKeys& k, bool
   int hist_chunk0 = 0;
   if (num_partitions <= kSwcMaxNum && g.nchunks_full > 0) {
     uint8_t* meta = (uint8_t*)scratch + l.pid_offset;
-    if (single) {
-      if (bits == 4) fb_rank_kernel<true, 4><<<g.nchunks_full, kRankBlock, 0, st>>>(k, dv, num_partitions, g, hist, meta);
-      else fb_rank_kernel<true, 8><<<g.nchunks_full, kRankBlock, 0, st>>>(k, dv, num_partitions, g, hist, meta);
+    const bool pow2 = (num_partitions & (num_partitions - 1)) == 0;
+#define FB_LAUNCH_RANK(S, B, P) \
+  fb_rank_kernel<S, B, P><<<g.nchunks_full, kRankBlock, 0, st>>>(k, dv, num_partitions, g, hist, meta)
+    if (single && pow2) {
+      if (bits == 4) FB_LAUNCH_RANK(true, 4, true);
+      else FB_LAUNCH_RANK(true, 8, true);
+    } else if (single) {
+      if (bits == 4) FB_LAUNCH_RANK(true, 4, false);
+      else FB_LAUNCH_RANK(true, 8, false);
     } else {
-      if (bits == 4) fb_rank_kernel<false, 4><<<g.nchunks_full, kRankBlock, 0, st>>>(k, dv, num_partitions, g, hist, meta);
-      else fb_rank_kernel<false, 8><<<g.nchunks_full, kRankBlock, 0, st>>>(k, dv, num_partitions, g, hist, meta);
+      if (bits == 4) FB_LAUNCH_RANK(false, 4, false);
+      else FB_LAUNCH_RANK(false, 8, false);
     }
+#undef FB_LAUNCH_RANK
     FB_CUDA(cudaGetLastError());
     hist_chunk0 = g.nchunks_full;
   }
